@@ -2,6 +2,7 @@
 """Benchmark of the fused flow hot path (contract: see the task statement / DESIGN.md section "Measurement").
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload q256|r64|m128] [--impl ours|reference]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch: ``Flow.log_prob`` on B rows followed by ``Flow.sample`` of
 B rows (inverse direction).  Default workload (BASELINE.json configs[2], the one the north-star target and the
@@ -201,6 +202,29 @@ def run_reference(args):
     print(json.dumps(line), flush=True)
 
 
+DUMP_BYTES = 48 << 20       # array data written by --dump-outputs, at most (plus a 128-byte header per .npy file)
+
+
+def dump_outputs(out_dir, outputs):
+    """Write the row-aligned outputs of the last timed step as <out_dir>/<name>.npy in float32.  When all of them
+    together exceed DUMP_BYTES, every output keeps the same rows: a sorted sample drawn from a private generator under
+    a fixed seed, so two runs with the same arguments write comparable files and torch's global RNG (which keys the
+    library's base draws) is left untouched."""
+    import numpy as np
+    import torch
+    rows = next(iter(outputs.values())).shape[0]
+    row_bytes = sum(4 * t[:1].numel() for t in outputs.values())
+    keep = min(rows, DUMP_BYTES // row_bytes)
+    idx = None
+    if keep < rows:
+        idx = torch.randperm(rows, generator=torch.Generator().manual_seed(0))[:keep].sort().values
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in outputs.items():
+        if idx is not None:
+            t = t[idx.to(t.device)]
+        np.save(os.path.join(out_dir, name + '.npy'), t.detach().float().cpu().numpy())
+
+
 def transformer_kernel_roofline(torch, dev, hbm_peak):
     """Stand-alone rational-quadratic spline transformer (b2f_transformer_apply, dense parameters): 16384 x 512 elements,
     (23 + 2) * 4 algorithmic bytes per element, CUDA-event timing over 10 launches, operands (771 MB of h) larger than L2."""
@@ -278,6 +302,8 @@ def run_ours(args):
         total_ms = ev[0].elapsed_time(ev[3 * args.steps])
         lp_ms = [ev[3 * i].elapsed_time(ev[3 * i + 1]) for i in range(args.steps)]
         s_ms = [ev[3 * i + 1].elapsed_time(ev[3 * i + 2]) for i in range(args.steps)]
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, {'log_prob': lp, 'sample': xs})
         del xs
         from torchflows_b200 import _native as N_
         flow.sample(4096, no_grad=True)
@@ -726,7 +752,14 @@ def main():
     ap.add_argument('--rows', type=int, default=0, help='override rows per GPU')
     ap.add_argument('--no-cpu', action='store_true', help='skip the cpu_baseline and gpu_eager_baseline legs')
     ap.add_argument('--no-fit', action='store_true', help='skip the Flow.fit probe (q256fit, w1024fit) of the default line')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write log_prob.npy and sample.npy of the last timed step (rank 0; a fixed row sample of '
+                         f'at most {DUMP_BYTES >> 20} MiB in all) to DIR')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and (args.impl != 'ours' or args.workload in ('w1024fit', 'q256fit')):
+        ap.error('--dump-outputs applies to the log_prob + sample workloads of --impl ours')
     args.warmup = max(args.warmup, 3) if args.impl == 'ours' else max(args.warmup, 1)
     if args.workload in ('w1024fit', 'q256fit'):
         run_fit(args)

@@ -10,6 +10,7 @@ and presets under fixed seeds, evaluates them on CPU in fp32, and stores inputs,
 (``state_dict``) and outputs.  The fixtures pin ``oracle/`` (tests/test_oracle_golden.py) and are the
 reference-produced half of the GPU parity tests (tests/test_gpu_*.py).
 """
+import io
 import os
 import sys
 import warnings
@@ -28,6 +29,39 @@ from torchflows.bijections.finite.autoregressive.transformers.spline.rational_qu
     RationalQuadratic)
 
 OUT = os.path.dirname(os.path.abspath(__file__))
+PART_BYTES = 900_000        # no file of the repository is larger than 1 MB
+
+
+def _nbytes(obj):
+    buf = io.BytesIO()
+    torch.save(obj, buf)
+    return buf.tell()
+
+
+def save(obj, name):
+    """torch.save(obj) as tests/golden/<name>; a list of cases (or a dict of such lists) larger than PART_BYTES goes to
+    numbered parts <stem>/00.pt, 01.pt, ... of whole cases instead, which tests/conftest.py (golden) joins back."""
+    path = os.path.join(OUT, name)
+    if _nbytes(obj) <= PART_BYTES:
+        torch.save(obj, path)
+        print(name, os.path.getsize(path) // 1024, 'KiB')
+        return
+    keys = list(obj) if isinstance(obj, dict) else [None]
+    items = [(k, c) for k in keys for c in (obj if k is None else obj[k])]
+    parts, size = [[]], 0
+    for k, c in items:
+        n = _nbytes(c)
+        if parts[-1] and size + n > PART_BYTES:
+            parts.append([])
+            size = 0
+        parts[-1].append((k, c))
+        size += n
+    stem = os.path.splitext(path)[0]
+    os.makedirs(stem, exist_ok=True)
+    for i, part in enumerate(parts):
+        out = [c for _, c in part] if keys == [None] else {k: [c for kk, c in part if kk == k] for k in keys}
+        torch.save(out, os.path.join(stem, f'{i:02d}.pt'))
+        print(f'{name} part {i:02d}', os.path.getsize(os.path.join(stem, f'{i:02d}.pt')) // 1024, 'KiB')
 
 
 def rq_bin_index(tr: RationalQuadratic, v, h, direction):
@@ -248,13 +282,11 @@ def context_cases():
 
 def main():
     torch.set_num_threads(1)   # fixed reduction order on the generating side
-    torch.save(transformer_cases(), os.path.join(OUT, 'transformers.pt'))
-    torch.save(preset_cases(), os.path.join(OUT, 'presets.pt'))
-    torch.save(grad_cases(), os.path.join(OUT, 'grads.pt'))
-    torch.save(fit_cases(), os.path.join(OUT, 'fit.pt'))
-    torch.save(context_cases(), os.path.join(OUT, 'context.pt'))
-    for f in ('transformers.pt', 'presets.pt', 'grads.pt', 'fit.pt', 'context.pt'):
-        print(f, os.path.getsize(os.path.join(OUT, f)) // 1024, 'KiB')
+    save(transformer_cases(), 'transformers.pt')
+    save(preset_cases(), 'presets.pt')
+    save(grad_cases(), 'grads.pt')
+    save(fit_cases(), 'fit.pt')
+    save(context_cases(), 'context.pt')
 
 
 if __name__ == '__main__':

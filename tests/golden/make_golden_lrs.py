@@ -25,7 +25,7 @@ from torchflows.bijections.finite.autoregressive import architectures as ref_arc
 from torchflows.bijections.finite.autoregressive.transformers.linear.affine import Scale  # noqa: E402
 from torchflows.bijections.finite.autoregressive.transformers.spline.linear_rational import LinearRational  # noqa: E402
 
-OUT = os.path.dirname(os.path.abspath(__file__))
+from make_golden import save  # noqa: E402
 
 
 def with_grads(tr, fn, v, h, g):
@@ -135,8 +135,7 @@ def layer_cases():
 
 def main():
     torch.manual_seed(0)
-    torch.save(dict(transformers=transformer_cases(), presets=preset_cases(), layers=layer_cases()), os.path.join(OUT, 'lrs.pt'))
-    print('wrote', os.path.join(OUT, 'lrs.pt'))
+    save(dict(transformers=transformer_cases(), presets=preset_cases(), layers=layer_cases()), 'lrs.pt')
 
 
 if __name__ == '__main__':

@@ -266,3 +266,29 @@ def test_philox_restatement_known_answer():
     from tests.test_gpu_sampling import philox4x32_10
     u = philox4x32_10(np.zeros(1, dtype=np.uint64), 0)
     assert [int(v[0]) for v in u] == [0x6627e8d5, 0xe169c58d, 0xbc57ac4c, 0x9b00dbd8]
+
+
+def test_bench_dump_outputs_fixed_row_sample(tmp_path):
+    """bench.py --dump-outputs: float32 .npy files within the size cap, the same seeded rows of every output in every
+    run, and torch's global RNG (which keys Flow.sample's draws) untouched."""
+    import numpy as np
+    import torch
+    import bench
+    g = torch.Generator().manual_seed(1)
+    rows, D = 2 * bench.DUMP_BYTES // (4 * 65), 64
+    lp, xs = torch.arange(rows, dtype=torch.float64), torch.randn(rows, D, generator=g)      # log_prob holds the row index
+    rng = torch.random.get_rng_state()
+    for d in ('a', 'b'):
+        bench.dump_outputs(str(tmp_path / d), {'log_prob': lp, 'sample': xs})
+    assert torch.equal(rng, torch.random.get_rng_state())
+    a_lp, a_xs = np.load(tmp_path / 'a' / 'log_prob.npy'), np.load(tmp_path / 'a' / 'sample.npy')
+    assert a_lp.dtype == a_xs.dtype == np.float32 and a_xs.shape[1] == D
+    assert 0 < len(a_lp) == len(a_xs) < rows
+    assert sum(f.stat().st_size for f in (tmp_path / 'a').iterdir()) <= bench.DUMP_BYTES + 1024
+    assert np.array_equal(a_lp, np.load(tmp_path / 'b' / 'log_prob.npy'))
+    assert np.array_equal(a_xs, np.load(tmp_path / 'b' / 'sample.npy'))
+    kept = a_lp.astype(np.int64)
+    assert np.all(np.diff(kept) > 0) and np.array_equal(xs.numpy()[kept], a_xs)
+    small = tmp_path / 'small'
+    bench.dump_outputs(str(small), {'log_prob': lp[:100], 'sample': xs[:100]})
+    assert np.array_equal(np.load(small / 'sample.npy'), xs[:100].numpy())
