@@ -34,9 +34,9 @@ enum b2f_transformer {
     B2F_T_AFFINE_INV = 3, /* Affine.inverse / InverseAffine.forward  x = (z-u1)/a, ld = -log a   affine.py:50-59 */
     B2F_T_RQ_FWD = 4,     /* RationalQuadratic.forward   spline/base.py:53-60, rational_quadratic.py:65-128 */
     B2F_T_RQ_INV = 5,     /* RationalQuadratic.inverse   spline/base.py:65-72, rational_quadratic.py:130-200 */
-    /* stand-alone transformer entry points only (b2f_transformer_apply / _backward), not flow programs: */
     B2F_T_LRS_FWD = 6,    /* LinearRational.forward      spline/linear_rational.py:92-135; 4 * n_bins parameters per element */
     B2F_T_LRS_INV = 7,    /* LinearRational.inverse      spline/linear_rational.py:137-182 */
+    /* stand-alone transformer entry points only (b2f_transformer_apply / _backward), not flow programs: */
     B2F_T_SCALE_FWD = 8,  /* Scale.forward               z = a*x, ld = +log a    affine.py:186-193 */
     B2F_T_SCALE_INV = 9   /* Scale.inverse               x = z/a, ld = -log a    affine.py:195-202 */
 };
@@ -55,6 +55,18 @@ enum b2f_op_kind {
     B2F_OP_MADE_SEQ = 4     /* the D-step sequential direction                      layers_base.py:213-223
                                as B2F_OP_MADE plus p[4] = int32 finalisation step of each hidden unit (H) */
 };
+
+/* (op kind, tkind, n_bins) combinations that flow programs accept (b2f_flow_apply, b2f_flow_sample, b2f_flow_apply_saving,
+ * b2f_flow_backward):
+ *   ELEMENTWISE           AFFINE_FWD / AFFINE_INV                                   n_bins ignored
+ *   COUPLING, MADE        SHIFT_*, AFFINE_*                                         n_bins ignored
+ *   COUPLING, MADE        RQ_FWD / RQ_INV, LRS_FWD / LRS_INV                        n_bins == 8, boundary > 0
+ *   MADE_SEQ              SHIFT_*, AFFINE_*                                         n_bins ignored
+ *   MADE_SEQ              RQ_FWD / RQ_INV, LRS_FWD / LRS_INV                        n_bins == 8, boundary > 0
+ *                         (b2f_flow_backward: RQ_INV / LRS_INV only, with B2F_FLAG_SEQ_LOGDET_EXACT)
+ * SCALE_* are stand-alone transformer kinds only.  Linear rational spline (LRS) programs run on the generic FP32 kernel
+ * (B2F_KERNEL_GENERIC); a MADE_SEQ LRS_INV layer with n_hidden <= 15 runs on the row-per-thread kernel (B2F_KERNEL_ROWS).
+ * The tensor-core kernels decline LRS ops. */
 
 /* W2 "tile layout": the reference's last Linear weight (Dt*P, H) (output index e*P+p, layers_base.py:143)
  * re-laid-out as [e][j][p] with p padded to PP = b2f_padded_params(P), so that the P parameters of one
@@ -140,8 +152,8 @@ typedef struct b2f_op {
     int32_t kind;     /* enum b2f_op_kind */
     int32_t tkind;    /* enum b2f_transformer */
     int32_t n_hidden; /* H */
-    int32_t n_bins;   /* RQ only (the fused program supports 8; b2f_transformer_apply supports 1..64) */
-    float boundary;   /* RQ only */
+    int32_t n_bins;   /* RQ / LRS only (flow programs support 8; b2f_transformer_apply supports 1..64) */
+    float boundary;   /* RQ / LRS only */
     int32_t flags;
     const void *p[6]; /* parameters, see enum b2f_op_kind */
     void *g[6];       /* b2f_flow_backward only: gradient buffers with the layout of p[i] (accumulated into) */

@@ -35,7 +35,13 @@ class LoweredOp:
 
 
 def params_per_element(tkind: int, n_bins: int) -> int:
+    if tkind in (N.T_LRS_FWD, N.T_LRS_INV):
+        return 4 * n_bins
     return {N.T_SHIFT_ADD: 1, N.T_SHIFT_SUB: 1, N.T_AFFINE_FWD: 2, N.T_AFFINE_INV: 2}.get(tkind, 3 * n_bins - 1)
+
+
+#: spline transformer kinds: their sequential MADE direction reports the reference's last-iteration log-det by default
+SPLINE_TKINDS = (N.T_RQ_FWD, N.T_RQ_INV, N.T_LRS_FWD, N.T_LRS_INV)
 
 
 def padded(P: int) -> int:
@@ -293,7 +299,7 @@ class FlowFunction(torch.autograd.Function):
         x2 = ctx.saved_tensors[0]
         ops = cfg.ops
         for op in ops:
-            if op.kind == N.OP_MADE_SEQ and op.tkind in (N.T_RQ_FWD, N.T_RQ_INV) and not (op.flags & N.FLAG_SEQ_LOGDET_EXACT):
+            if op.kind == N.OP_MADE_SEQ and op.tkind in SPLINE_TKINDS and not (op.flags & N.FLAG_SEQ_LOGDET_EXACT):
                 raise NotImplementedError(
                     'gradients through the sequential direction of a spline MADE layer are implemented for the exact '
                     'log-determinant only: set layer.sequential_log_det_reference_quirk = False (the reference returns '
@@ -393,7 +399,7 @@ def run_program(ops: Sequence[LoweredOp], x2: torch.Tensor, want_log_prob=False,
         # The reference's last-iteration log-det of a sequential spline layer (SURVEY Appendix B.3) has no fused gradient:
         # when gradients are needed the layer is lowered with the exact log-determinant instead (same value to ~1e-5 at
         # initialisation, a well-defined objective afterwards), so that fit() / variational_fit() work out of the box.
-        quirky = [i for i, op in enumerate(ops) if op.kind == N.OP_MADE_SEQ and op.tkind in (N.T_RQ_FWD, N.T_RQ_INV)
+        quirky = [i for i, op in enumerate(ops) if op.kind == N.OP_MADE_SEQ and op.tkind in SPLINE_TKINDS
                   and not (op.flags & N.FLAG_SEQ_LOGDET_EXACT)]
         if quirky:
             global _warned_seq_exact

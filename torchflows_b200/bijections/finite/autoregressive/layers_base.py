@@ -2,9 +2,10 @@
 
 Each class pairs a conditioner with a transformer like the reference, and adds ``lower(direction)``: the
 description of the layer as one op of a fused libb2f flow program (conditioner GEMMs + transformer + log-det
-in one kernel, ``h`` never written to HBM).  Configurations outside the fused path (non-default conditioner
-depth / nonlinearity, globally learned parameter subsets, n_bins != 8) are detected at construction time and run
-as a *composite*: conditioner as library GEMMs, transformer as the stand-alone transformer kernel."""
+in one kernel, ``h`` never written to HBM).  Rational-quadratic and linear rational splines with n_bins = 8 are fused
+like the affine transformers.  Configurations outside the fused path (non-default conditioner depth / nonlinearity,
+globally learned parameter subsets, n_bins != 8) are detected at construction time and run as a *composite*:
+conditioner as library GEMMs, transformer as the stand-alone transformer kernel."""
 import os
 from typing import Any, List, Optional, Tuple, Type, Union
 
@@ -20,6 +21,7 @@ from torchflows_b200.bijections.finite.autoregressive.conditioning.coupling_mask
 from torchflows_b200.bijections.finite.autoregressive.conditioning.transforms import (MADE, ConditionerTransform,
                                                                                        FeedForward, Linear)
 from torchflows_b200.bijections.finite.autoregressive.transformers.base import ScalarTransformer, TensorTransformer
+from torchflows_b200.bijections.finite.autoregressive.transformers.spline.linear_rational import LinearRational
 from torchflows_b200.bijections.finite.autoregressive.transformers.spline.rational_quadratic import RationalQuadratic
 from torchflows_b200.utils import flatten_event, get_batch_shape, unflatten_event
 
@@ -92,9 +94,9 @@ def _fits_fused_kernel(n_dim: int, n_hidden: int, kind: int = N.OP_ELEMENTWISE, 
 
 
 def _transformer_fusable(tr) -> bool:
-    if isinstance(tr, RationalQuadratic):
+    if isinstance(tr, (RationalQuadratic, LinearRational)):
         return tr.n_bins == 8
-    # Affine / InverseAffine / Shift; LinearRational and Scale have stand-alone kernels only (kinds above T_RQ_INV)
+    # Affine / InverseAffine / Shift; Scale has stand-alone kernels only
     return isinstance(tr, ScalarTransformer) and 0 <= tr._tkind_forward <= N.T_RQ_INV
 
 
@@ -119,7 +121,7 @@ class AutoregressiveBijection(Bijection):
 
     def _spline_args(self):
         tr = self.transformer
-        return (tr.n_bins, tr.boundary) if isinstance(tr, RationalQuadratic) else (0, 0.0)
+        return (tr.n_bins, tr.boundary) if isinstance(tr, (RationalQuadratic, LinearRational)) else (0, 0.0)
 
 
 class CouplingBijection(AutoregressiveBijection):
@@ -317,8 +319,8 @@ class MaskedAutoregressiveBijection(AutoregressiveBijection):
         if not (ct.n_layers == 2 and ct.is_plain and isinstance(transformer, ScalarTransformer)):
             raise NotImplementedError('masked autoregressive layers are implemented for the default MADE depth '
                                       '(n_layers=2) and predicted parameters only')
-        # transformers without a whole-flow kernel (LinearRational, splines with n_bins != 8) run as a composite: masked
-        # conditioner GEMMs + the stand-alone transformer kernel, the sequential direction as the reference's D-step loop
+        # transformers without a whole-flow kernel (splines with n_bins != 8) run as a composite: masked conditioner
+        # GEMMs + the stand-alone transformer kernel, the sequential direction as the reference's D-step loop
         # With a context, MADE concatenates it to x and gives the context columns degrees n_dim+1.. (transforms.py:
         # 222-226).  Hidden units that see a context column therefore have a degree > n_dim, and the strict output mask
         # (transforms.py:254) cuts every such unit off from every output: the context provably never reaches h.  The
@@ -332,8 +334,11 @@ class MaskedAutoregressiveBijection(AutoregressiveBijection):
         fin = ct.sequential[0].mask[:, :self.n_dim].sum(dim=1).to(torch.int32)
         self.register_buffer('_fin_steps', fin, persistent=False)
         # event sizes whose backward tile no longer fits shared memory (D >= 768) run as a composite, see _composite_*
-        self._fusable = _transformer_fusable(transformer) and _fits_fused_kernel(
-            self.n_dim, ct.n_hidden, N.OP_MADE, transformer._tkind_forward, self._spline_args()[0])
+        # (linear rational spline layers with a context stay composite)
+        self._fusable = (_transformer_fusable(transformer)
+                         and not (isinstance(transformer, LinearRational) and self._n_context_cols > 0)
+                         and _fits_fused_kernel(self.n_dim, ct.n_hidden, N.OP_MADE, transformer._tkind_forward,
+                                                self._spline_args()[0]))
 
     def _lower(self, one_pass: bool, transformer_direction: str):
         seq = self.conditioner_transform.sequential

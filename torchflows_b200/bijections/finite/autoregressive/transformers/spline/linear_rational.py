@@ -5,7 +5,9 @@ Per element 4K parameters: u_x = h[:K] (width logits), u_y = h[K:2K] (heights ar
 u_lambda = h[2K:3K] (position of the intermediate knot inside each bin, through a sigmoid), u_d = h[3K:4K-1] (interior
 derivative logits, /100, edges fixed at 1), u_w0 = h[4K-1] (weight of the first knot).  Forward, inverse and backward are one
 kernel launch each (csrc/b2f_transformer.cu, math in csrc/b2f_lrs.cuh) instead of ~90 ATen launches and a boolean-mask copy of
-h; layers built on it run as a composite (conditioner GEMMs + this kernel), not inside the whole-flow kernels."""
+h.  With the default n_bins = 8 (32 parameters per element), coupling and MADE layers built on it are ops of fused flow programs:
+the same device math runs inside the whole-flow kernels, one launch per direction, the sequential MADE direction included, and
+one fused backward.  Other bin counts run as a composite (conditioner GEMMs + the stand-alone kernel)."""
 import math
 from typing import Tuple, Union
 

@@ -54,6 +54,8 @@ __device__ __forceinline__ void run_transform(const Tile& t, const DevOp& op, in
         B2F_CASE(B2F_T_AFFINE_INV)
         B2F_CASE(B2F_T_RQ_FWD)
         B2F_CASE(B2F_T_RQ_INV)
+        B2F_CASE(B2F_T_LRS_FWD)
+        B2F_CASE(B2F_T_LRS_INV)
     }
 #undef B2F_CASE
 }
@@ -248,7 +250,8 @@ static int flow_apply_impl(const b2f_op_t* ops, int32_t n_ops, const float* x, f
     {
         // Spline programs (23 parameters per element: the output layer is a real GEMM) go to the tcgen05 kernel first,
         // affine / shift programs and anything with a sequential layer to the row-per-thread kernel first; what neither
-        // takes runs on the generic kernel below.
+        // takes runs on the generic kernel below.  Linear rational spline programs are not RQ programs here: every
+        // tensor-core kernel declines them by transformer kind, the row-per-thread kernel takes their sequential inverse.
         bool has_rq = false;
         for (int i = 0; i < n_ops; ++i)
             if (ops[i].kind >= B2F_OP_COUPLING && (ops[i].tkind == B2F_T_RQ_FWD || ops[i].tkind == B2F_T_RQ_INV)) has_rq = true;
@@ -280,7 +283,7 @@ static int flow_apply_impl(const b2f_op_t* ops, int32_t n_ops, const float* x, f
                         "which only the row-per-thread kernel takes, and that kernel declined this program", i);
     FlowArgs A;
     memset(&A, 0, sizeof(A));
-    int Hmax = 1, has_seq = 0, has_rq = 0;
+    int Hmax = 1, has_seq = 0, has_spline = 0;
     for (int i = 0; i < n_ops; ++i) {
         const b2f_op_t& o = ops[i];
         DevOp& d = A.ops[i];
@@ -299,14 +302,19 @@ static int flow_apply_impl(const b2f_op_t* ops, int32_t n_ops, const float* x, f
                     return fail(B2F_ERR_INVALID, "op %d: conditioner parameters missing", i);
                 if (params_per_element(o.tkind, 8) < 0) return fail(B2F_ERR_INVALID, "op %d: transformer kind", i);
                 const bool rq = o.tkind == B2F_T_RQ_FWD || o.tkind == B2F_T_RQ_INV;
+                const bool lrs = o.tkind == B2F_T_LRS_FWD || o.tkind == B2F_T_LRS_INV;
+                if (o.tkind == B2F_T_SCALE_FWD || o.tkind == B2F_T_SCALE_INV)
+                    return fail(B2F_ERR_UNSUPPORTED, "op %d: transformer kind %d has no flow-program kernel", i, o.tkind);
                 if (rq && o.n_bins != 8)
                     return fail(B2F_ERR_UNSUPPORTED, "op %d: fused RQ spline needs n_bins == 8 (got %d)", i, o.n_bins);
-                if (rq && !(o.boundary > 0.0f)) return fail(B2F_ERR_INVALID, "op %d: boundary", i);
+                if (lrs && o.n_bins != 8)
+                    return fail(B2F_ERR_UNSUPPORTED, "op %d: fused linear rational spline needs n_bins == 8 (got %d)", i, o.n_bins);
+                if ((rq || lrs) && !(o.boundary > 0.0f)) return fail(B2F_ERR_INVALID, "op %d: boundary", i);
                 if (o.kind == B2F_OP_COUPLING && D < 2) return fail(B2F_ERR_INVALID, "op %d: coupling needs D >= 2", i);
                 if (o.kind == B2F_OP_MADE_SEQ) { if (!o.p[4]) return fail(B2F_ERR_INVALID, "op %d: finalisation steps", i); has_seq = 1; }
-                if (rq && (reinterpret_cast<uintptr_t>(o.p[2]) & 15))
+                if ((rq || lrs) && (reinterpret_cast<uintptr_t>(o.p[2]) & 15))
                     return fail(B2F_ERR_INVALID, "op %d: W2 tile layout must be 16-byte aligned", i);
-                has_rq |= rq;
+                has_spline |= rq || lrs;
                 Hmax = std::max(Hmax, o.n_hidden);
                 break;
             }
@@ -320,7 +328,7 @@ static int flow_apply_impl(const b2f_op_t* ops, int32_t n_ops, const float* x, f
     int TM, NT;
     if (has_seq) { TM = 64; NT = 64; }          // sequential op: thread == sample, every warp busy
     else if (D <= 32) { TM = 128; NT = 256; }
-    else { TM = 64; NT = has_rq ? 512 : 256; }
+    else { TM = 64; NT = has_spline ? 512 : 256; }
     if (const char* e = getenv("B2F_TM")) TM = atoi(e);
     if (const char* e = getenv("B2F_NT")) NT = atoi(e);
     auto smem_bytes = [&](int tm, int nt) {

@@ -3,7 +3,7 @@
 // Replaces torch autograd through the ~470-op graph the reference builds for one log_prob call
 // (/root/reference/torchflows/flows.py:199-224 -> bijections/base.py:203-224 -> layers_base.py:145-153,
 //  202-211, 300-318 -> transforms.py:293-307 -> transformers/...).  The math of the transformer backward is
-// SURVEY.md Appendix D (csrc/b2f_math.cuh: rq_backward_fwd, affine_*_backward).
+// SURVEY.md Appendix D (csrc/b2f_math.cuh: rq_backward_fwd, affine_*_backward; csrc/b2f_lrs.cuh: lrs_backward).
 //
 // Per CTA (tile of TM samples, both the activation tile xt and the gradient tile gt live in shared memory):
 //   phase A  recompute the forward pass layer by layer; the tile as it enters each conditioner layer is written
@@ -34,7 +34,7 @@ struct BwdOp {
 
 struct BwdArgs {
     BwdOp ops[B2F_MAX_OPS];
-    int n_ops, D, TM, logTM, XS, HS, WPG, G, flags, wst_stride;
+    int n_ops, D, TM, logTM, XS, HS, WPG, G, flags, wst_stride, dhs_pp;
     long long B;
     const float* x;
     const float* gy;
@@ -52,7 +52,7 @@ struct BTile {
     float* dhid;  // [TM][HS] gradient w.r.t. hidden activations, then pre-activations
     float* dhp;   // [WPG][TM][HS] per-slot partial sums of dhid (a warp owns its (slot, 32 samples) slice: no atomics)
     float* GL;    // [TM]     dL/dlog_det of each sample (constant through the layers)
-    float* dhs;   // [NW][32][PPmax] per-warp staging of dL/dh for the weight-gradient product
+    float* dhs;   // [NW][32][dhs_pp] per-warp staging of dL/dh for the weight-gradient product (dhs_pp >= every PP)
     float* wst;   // [NW][2][wst_stride] per-warp double buffer of one element's output-layer weights (spline layers)
     int rows, precise, wst_stride;
 };
@@ -76,6 +76,10 @@ __device__ __forceinline__ void transformer_backward_element(float v, const floa
             auto g = [&](int i, float val) { dh[i] = val; };
             rq_backward_fwd<8, MODE>(v, h, 8, boundary, GZ, GL, dv, g);
         }
+    } else if constexpr (TK == B2F_T_LRS_FWD || TK == B2F_T_LRS_INV) {
+        auto h = [&](int i) { return acc[i]; };
+        auto g = [&](int i, float val) { dh[i] = val; };
+        lrs_backward<8, TK == B2F_T_LRS_INV>(v, h, 8, boundary, GZ, GL, dv, g);
     } else {
         auto h = [&](int i) { return acc[i]; };
         auto g = [&](int i, float val) { dh[i] = val; };
@@ -450,6 +454,8 @@ __device__ __forceinline__ void run_transform_backward(const BTile& b, const Bwd
         case B2F_T_AFFINE_INV: transform_pass_backward<B2F_T_AFFINE_INV, MODE>(b, op, t0, n_tgt); break;
         case B2F_T_RQ_FWD: transform_pass_backward_rq<B2F_T_RQ_FWD, MODE>(b, op, t0, n_tgt); break;
         case B2F_T_RQ_INV: transform_pass_backward_rq<B2F_T_RQ_INV, MODE>(b, op, t0, n_tgt); break;
+        case B2F_T_LRS_FWD: transform_pass_backward<B2F_T_LRS_FWD, MODE>(b, op, t0, n_tgt); break;
+        case B2F_T_LRS_INV: transform_pass_backward<B2F_T_LRS_INV, MODE>(b, op, t0, n_tgt); break;
         default: break;
     }
 }
@@ -462,6 +468,7 @@ __device__ __forceinline__ void run_sequential_backward(const BTile& b, const Bw
         case B2F_T_AFFINE_FWD: sequential_pass_backward<B2F_T_AFFINE_FWD, MODE>(b, op, z_saved); break;
         case B2F_T_AFFINE_INV: sequential_pass_backward<B2F_T_AFFINE_INV, MODE>(b, op, z_saved); break;
         case B2F_T_RQ_INV: sequential_pass_backward<B2F_T_RQ_INV, MODE>(b, op, z_saved); break;
+        case B2F_T_LRS_INV: sequential_pass_backward<B2F_T_LRS_INV, MODE>(b, op, z_saved); break;
         default: break;
     }
 }
@@ -474,6 +481,7 @@ __device__ __forceinline__ void run_sequential_forward(const Tile& t, const DevO
         case B2F_T_AFFINE_FWD: sequential_pass<B2F_T_AFFINE_FWD, MODE>(t, op); break;
         case B2F_T_AFFINE_INV: sequential_pass<B2F_T_AFFINE_INV, MODE>(t, op); break;
         case B2F_T_RQ_INV: sequential_pass<B2F_T_RQ_INV, MODE>(t, op); break;
+        case B2F_T_LRS_INV: sequential_pass<B2F_T_LRS_INV, MODE>(t, op); break;
         default: break;
     }
 }
@@ -487,6 +495,8 @@ __device__ __forceinline__ void run_transform_forward(const Tile& t, const DevOp
         case B2F_T_AFFINE_INV: transform_pass<B2F_T_AFFINE_INV, MODE>(t, op, t0, n_tgt); break;
         case B2F_T_RQ_FWD: transform_pass<B2F_T_RQ_FWD, MODE>(t, op, t0, n_tgt); break;
         case B2F_T_RQ_INV: transform_pass<B2F_T_RQ_INV, MODE>(t, op, t0, n_tgt); break;
+        case B2F_T_LRS_FWD: transform_pass<B2F_T_LRS_FWD, MODE>(t, op, t0, n_tgt); break;
+        case B2F_T_LRS_INV: transform_pass<B2F_T_LRS_INV, MODE>(t, op, t0, n_tgt); break;
         default: break;
     }
 }
@@ -517,8 +527,8 @@ __global__ void __launch_bounds__(384) flow_backward_kernel(const __grid_constan
     t.ldp = b.dhid + TM * HS;              // [WPG][TM] (written by the forward recompute, unused)
     b.GL = t.ldp + A.WPG * TM;             // [TM]
     float* ea = b.GL + TM;                 // [3*D]
-    b.dhs = ea + ((3 * D + 3) & ~3);       // [NW][32][24], 16-byte aligned
-    b.dhp = b.dhs + NW * 32 * 24;          // [WPG][TM][HS]
+    b.dhs = ea + ((3 * D + 3) & ~3);       // [NW][32][dhs_pp], 16-byte aligned
+    b.dhp = b.dhs + NW * 32 * A.dhs_pp;    // [WPG][TM][HS]
     b.wst = b.dhp + ((A.WPG * TM * HS + 3) & ~3);
     b.wst_stride = A.wst_stride;
     const long long row0 = (long long)blockIdx.x * TM;
@@ -781,7 +791,16 @@ static int ilog2b(int v) { int l = 0; while ((1 << l) < v) ++l; return l; }
 // element's output-layer weights per warp (wst_stride > 0: tensor-core path).  Preferred shapes first, then smaller ones
 // (fewer warps, then without the weight staging) until the shared-memory footprint fits; false if nothing fits.
 // b2f_flow_backward_fits() answers the same question for callers that must decide before building a program.
-struct BwdShape { int TM, NT, wst_stride; size_t smem; };
+struct BwdShape { int TM, NT, wst_stride, dhs_pp; size_t smem; };
+
+// padded parameters per element of the widest transformer of a program: 32 with a linear rational spline, else 24
+static int bwd_dhs_pp(const b2f_op_t* ops, int32_t n_ops) {
+    for (int i = 0; i < n_ops; ++i)
+        if ((ops[i].kind == B2F_OP_COUPLING || ops[i].kind == B2F_OP_MADE || ops[i].kind == B2F_OP_MADE_SEQ) &&
+            (ops[i].tkind == B2F_T_LRS_FWD || ops[i].tkind == B2F_T_LRS_INV))
+            return 32;
+    return 24;
+}
 
 static bool bwd_tile_shape(const b2f_op_t* ops, int32_t n_ops, int32_t D, int32_t flags, BwdShape& out) {
     int Hmax = 1, Hrq = 0;
@@ -795,12 +814,12 @@ static bool bwd_tile_shape(const b2f_op_t* ops, int32_t n_ops, int32_t D, int32_
             if (reinterpret_cast<uintptr_t>(o.p[2]) & 15) rq_aligned = false;
         }
     }
-    const int XS = D | 1, HS = Hmax | 1;
+    const int XS = D | 1, HS = Hmax | 1, dhs_pp = bwd_dhs_pp(ops, n_ops);
     const int wst_pref = (Hrq > 0 && rq_aligned && !(flags & B2F_FLOW_MODE_PRECISE)) ? ((Hrq * 24 + 24 + 3) & ~3) : 0;
     auto smem_bytes = [&](int tm, int nt, int wst) {
         const int wpg = (nt / 32) / (tm / 32);
         return (size_t)sizeof(float) * (2 * (size_t)tm * XS + 2 * (size_t)tm * HS + (((size_t)wpg * tm * HS + 3) & ~3) +
-                                        (size_t)wpg * tm + tm + ((3 * D + 3) & ~3) + (size_t)(nt / 32) * 32 * 24 +
+                                        (size_t)wpg * tm + tm + ((3 * D + 3) & ~3) + (size_t)(nt / 32) * 32 * dhs_pp +
                                         (size_t)(nt / 32) * 2 * wst + 4);
     };
     // spline programs: 12 warps on one 32-row tile (the kernel is latency-bound: measured 10.4 ms against 11.6 ms for
@@ -818,7 +837,7 @@ static bool bwd_tile_shape(const b2f_op_t* ops, int32_t n_ops, int32_t D, int32_
             if (TM < 32 || (TM & (TM - 1)) || NT % 32 || NT > 384 || (NT / 32) % (TM / 32) || NT / 32 < TM / 32) continue;
             const size_t smem = smem_bytes(TM, NT, tries[i].wst);
             if (smem > limit) continue;
-            out.TM = TM; out.NT = NT; out.wst_stride = tries[i].wst; out.smem = smem;
+            out.TM = TM; out.NT = NT; out.wst_stride = tries[i].wst; out.dhs_pp = dhs_pp; out.smem = smem;
             return true;
         }
     return false;
@@ -873,6 +892,12 @@ extern "C" int b2f_flow_backward(const b2f_op_t* ops, int32_t n_ops, const float
                     return fail(B2F_ERR_INVALID, "op %d: conditioner parameters missing", i);
                 if ((o.tkind == B2F_T_RQ_FWD || o.tkind == B2F_T_RQ_INV) && o.n_bins != 8)
                     return fail(B2F_ERR_UNSUPPORTED, "op %d: fused RQ spline needs n_bins == 8", i);
+                if ((o.tkind == B2F_T_LRS_FWD || o.tkind == B2F_T_LRS_INV) && (o.n_bins != 8 || !(o.boundary > 0.0f)))
+                    return fail(B2F_ERR_UNSUPPORTED, "op %d: fused linear rational spline needs n_bins == 8 and a boundary", i);
+                if (o.tkind != B2F_T_SHIFT_ADD && o.tkind != B2F_T_SHIFT_SUB && o.tkind != B2F_T_AFFINE_FWD &&
+                    o.tkind != B2F_T_AFFINE_INV && o.tkind != B2F_T_RQ_FWD && o.tkind != B2F_T_RQ_INV &&
+                    o.tkind != B2F_T_LRS_FWD && o.tkind != B2F_T_LRS_INV)
+                    return fail(B2F_ERR_UNSUPPORTED, "op %d: transformer kind %d has no fused backward", i, o.tkind);
                 const bool any_g = o.g[0] || o.g[1] || o.g[2] || o.g[3];
                 if (any_g && !(o.g[0] && o.g[1] && o.g[2] && o.g[3]))
                     return fail(B2F_ERR_INVALID, "op %d: give all four gradient buffers or none", i);
@@ -885,8 +910,15 @@ extern "C" int b2f_flow_backward(const b2f_op_t* ops, int32_t n_ops, const float
             case B2F_OP_MADE_SEQ: {
                 if (!o.p[0] || !o.p[1] || !o.p[2] || !o.p[3] || !o.p[4] || o.n_hidden <= 0)
                     return fail(B2F_ERR_INVALID, "op %d: conditioner parameters missing", i);
-                const bool rq = o.tkind == B2F_T_RQ_INV || o.tkind == B2F_T_RQ_FWD;
-                if (o.tkind == B2F_T_RQ_FWD) return fail(B2F_ERR_UNSUPPORTED, "op %d: sequential forward spline", i);
+                const bool rq = o.tkind == B2F_T_RQ_INV || o.tkind == B2F_T_RQ_FWD || o.tkind == B2F_T_LRS_INV ||
+                                o.tkind == B2F_T_LRS_FWD;
+                if (o.tkind == B2F_T_RQ_FWD || o.tkind == B2F_T_LRS_FWD)
+                    return fail(B2F_ERR_UNSUPPORTED, "op %d: sequential forward spline", i);
+                if (o.tkind != B2F_T_SHIFT_ADD && o.tkind != B2F_T_SHIFT_SUB && o.tkind != B2F_T_AFFINE_FWD &&
+                    o.tkind != B2F_T_AFFINE_INV && !rq)
+                    return fail(B2F_ERR_UNSUPPORTED, "op %d: transformer kind %d has no fused backward", i, o.tkind);
+                if (o.tkind == B2F_T_LRS_INV && !(o.boundary > 0.0f))
+                    return fail(B2F_ERR_UNSUPPORTED, "op %d: linear rational spline needs a boundary", i);
                 if (rq && (o.n_bins != 8 || !(o.flags & B2F_FLAG_SEQ_LOGDET_EXACT)))
                     return fail(B2F_ERR_UNSUPPORTED,
                                 "op %d: the backward of a sequential spline layer needs B2F_FLAG_SEQ_LOGDET_EXACT (the "
@@ -920,6 +952,7 @@ extern "C" int b2f_flow_backward(const b2f_op_t* ops, int32_t n_ops, const float
     if (!bwd_tile_shape(ops, n_ops, D, A.flags, shape))
         return fail(B2F_ERR_UNSUPPORTED, "b2f_flow_backward: D=%d H=%d does not fit shared memory", D, Hmax);
     A.wst_stride = shape.wst_stride;
+    A.dhs_pp = shape.dhs_pp;
     const int TM = shape.TM, NT = shape.NT;
     const size_t smem = shape.smem;
     A.TM = TM; A.logTM = ilog2b(TM); A.G = TM / 32; A.WPG = (NT / 32) / A.G;

@@ -4,6 +4,7 @@
 #pragma once
 #include "b2f_common.cuh"
 #include "b2f_math.cuh"
+#include "b2f_lrs.cuh"
 
 namespace b2f {
 
@@ -22,6 +23,11 @@ template <> struct TInfo<B2F_T_AFFINE_FWD> { static constexpr int P = 2, PP = 2;
 template <> struct TInfo<B2F_T_AFFINE_INV> { static constexpr int P = 2, PP = 2; };
 template <> struct TInfo<B2F_T_RQ_FWD> { static constexpr int P = 23, PP = 24; };
 template <> struct TInfo<B2F_T_RQ_INV> { static constexpr int P = 23, PP = 24; };
+template <> struct TInfo<B2F_T_LRS_FWD> { static constexpr int P = 32, PP = 32; };     // LinearRational, n_bins 8: 4 * 8
+template <> struct TInfo<B2F_T_LRS_INV> { static constexpr int P = 32, PP = 32; };
+
+// transformer kinds whose sequential direction reports the reference's last-iteration log-det (SURVEY Appendix B.3)
+template <int TK> constexpr bool kSplineTk = TK == B2F_T_RQ_FWD || TK == B2F_T_RQ_INV || TK == B2F_T_LRS_FWD || TK == B2F_T_LRS_INV;
 
 // transformer parameters of one element from the hidden activations of this thread's sample:
 // acc[p] = b2[e*P+p] + sum_j W2tile[e][j][p] * hid[j]          (transforms.py:297-300, last Linear)
@@ -67,7 +73,11 @@ __device__ __forceinline__ void transform_element(float v, const float (&acc)[PP
     else if constexpr (TK == B2F_T_SHIFT_SUB) { out = v - acc[0]; ld = 0.0f; }
     else if constexpr (TK == B2F_T_AFFINE_FWD) affine_fwd<MODE>(v, acc[0], acc[1], out, ld);
     else if constexpr (TK == B2F_T_AFFINE_INV) affine_inv<MODE>(v, acc[0], acc[1], out, ld);
-    else {
+    else if constexpr (TK == B2F_T_LRS_FWD || TK == B2F_T_LRS_INV) {
+        // linear rational spline (csrc/b2f_lrs.cuh): libm arithmetic in every mode
+        auto h = [&](int i) { return acc[i]; };
+        lrs_apply<8, TK == B2F_T_LRS_INV>(v, h, 8, boundary, out, ld);
+    } else {
         int k;
         auto h = [&](int i) { return acc[i]; };
         rq_apply<8, TK == B2F_T_RQ_INV, MODE>(v, h, 8, boundary, out, ld, k);
@@ -155,7 +165,7 @@ __device__ __forceinline__ void sequential_pass(const Tile& t, const DevOp& op) 
     float* act = t.act + m * t.HS;
     float* xr = t.xt + m * t.XS;
     for (int j = 0; j < H; ++j) { pre[j] = __ldg(op.p1 + j); act[j] = 0.0f; }
-    const bool quirk = (TK == B2F_T_RQ_INV || TK == B2F_T_RQ_FWD) && !(op.flags & B2F_FLAG_SEQ_LOGDET_EXACT);
+    const bool quirk = kSplineTk<TK> && !(op.flags & B2F_FLAG_SEQ_LOGDET_EXACT);
     float ldsum = 0.0f;
     for (int i = 0; i < D; ++i) {
         // hidden units whose inputs x_0..x_{i-1} are now all final

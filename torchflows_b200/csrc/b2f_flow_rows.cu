@@ -34,7 +34,7 @@ int try_launch_flow_rows(const b2f_op_t* ops, int32_t n_ops, const float* x, flo
     if ((reinterpret_cast<uintptr_t>(x) & 15) || (y && (reinterpret_cast<uintptr_t>(y) & 15))) return 0;
     RowsArgs A;
     memset(&A, 0, sizeof(A));
-    int Hmax = 0, Hrq = 0, n_runs = 0, n_cond = 0;
+    int Hmax = 0, Hrq = 0, n_runs = 0, n_cond = 0, wst_floats = 0;
     bool prev_ew = false;
     for (int i = 0; i < n_ops; ++i) {
         const b2f_op_t& o = ops[i];
@@ -54,12 +54,15 @@ int try_launch_flow_rows(const b2f_op_t* ops, int32_t n_ops, const float* x, flo
                 if (!o.p[0] || !o.p[1] || !o.p[2] || !o.p[3] || o.n_hidden <= 0 || o.n_hidden > 32) return 0;
                 if (o.flags & B2F_FLAG_ROW_BIAS) return 0;      // context-conditioned layers: generic kernel
                 if (o.kind == B2F_OP_MADE_SEQ && !o.p[4]) return 0;
-                if (o.tkind == B2F_T_RQ_FWD || o.tkind == B2F_T_RQ_INV) {
+                if (o.tkind == B2F_T_RQ_FWD || o.tkind == B2F_T_RQ_INV || o.tkind == B2F_T_LRS_INV) {
                     // splines: only the D-step sequential direction (the one-pass direction has a real GEMM as its output
-                    // layer and belongs on the tensor cores)
+                    // layer and belongs on the tensor cores, or for the linear rational spline on the generic kernel)
                     if (o.kind != B2F_OP_MADE_SEQ || o.n_bins != 8 || !(o.boundary > 0.0f) || o.n_hidden > 15) return 0;
                     if (reinterpret_cast<uintptr_t>(o.p[2]) & 15) return 0;
+                    if (o.tkind == B2F_T_LRS_INV && (o.flags & B2F_FLAG_SEQ_FOLDED)) return 0;    // no folded variant
                     Hrq = std::max(Hrq, o.n_hidden);
+                    wst_floats = std::max(wst_floats, o.n_hidden * padded_params(params_per_element(o.tkind, 8)) +
+                                                          padded_params(params_per_element(o.tkind, 8)));
                 } else if (o.tkind != B2F_T_SHIFT_ADD && o.tkind != B2F_T_SHIFT_SUB && o.tkind != B2F_T_AFFINE_FWD &&
                            o.tkind != B2F_T_AFFINE_INV) {
                     return 0;
@@ -85,7 +88,7 @@ int try_launch_flow_rows(const b2f_op_t* ops, int32_t n_ops, const float* x, flo
         const b2f_op_t& o = ops[i];
         if (o.kind != B2F_OP_COUPLING && o.kind != B2F_OP_MADE && o.kind != B2F_OP_MADE_SEQ) continue;
         const int n_src = o.kind == B2F_OP_COUPLING ? D / 2 : D, n_tgt = o.kind == B2F_OP_COUPLING ? D - D / 2 : D;
-        const bool rq = o.tkind == B2F_T_RQ_FWD || o.tkind == B2F_T_RQ_INV;
+        const bool rq = o.tkind == B2F_T_RQ_FWD || o.tkind == B2F_T_RQ_INV || o.tkind == B2F_T_LRS_INV;
         const int P = (o.tkind == B2F_T_SHIFT_ADD || o.tkind == B2F_T_SHIFT_SUB) ? 1 : 2;
         A.woff[i] = (int)wtotal;
         wtotal += (size_t)n_src * HP + HP + (rq ? 0 : (size_t)n_tgt * P * HP);
@@ -114,7 +117,7 @@ int try_launch_flow_rows(const b2f_op_t* ops, int32_t n_ops, const float* x, flo
         if (ctas * (NT / 32) >= 16) inplace = false;
     }
     if (inplace) XS = 0;                                           // no tile
-    const int rq_stride = spline ? ((Hrq * 24 + 24 + 3) & ~3) : 0;
+    const int rq_stride = spline ? ((wst_floats + 3) & ~3) : 0;     // one element's output-layer block: H * PP + PP floats
     auto smem_for = [&](int nt) {
         return sizeof(float) * ((size_t)(nt / 32) * 32 * R * XS + (size_t)n_runs * 2 * D + 2 * D + std::max(8, 2 * (nt / 32)) +
                                 wtotal + (size_t)(nt / 32) * 2 * rq_stride);        // (+ [2][warps] partials, >= 8 floats)

@@ -125,7 +125,7 @@ __device__ __forceinline__ void stage_weights(float* wbuf, const DevOp& op, int 
         }
     }
     if (tid < HP) b1[tid] = (tid < H) ? __ldg(op.p1 + tid) : 0.0f;
-    if constexpr (P > 2) return;        // spline layers: the output layer (23 x H per element) is streamed per element
+    if constexpr (P > 2) return;        // spline layers: the output layer (P x H per element) is streamed per element
     for (int d = tid; d < n_tgt * P * HP; d += kRowsThreads) {
         const int q = d / HP, j = d - q * HP, ep = q / P, p = q - ep * P;
         const int e = f ? n_tgt - 1 - ep : ep;
@@ -299,10 +299,11 @@ __device__ __forceinline__ void rows_sequential(float* x0, int XS, int D, const 
     }
 }
 
-// The same D-step sequential direction for a SPLINE masked autoregressive layer (MaskedAutoregressiveRQNSF sampling,
-// InverseAutoregressiveRQNSF density).  The output layer is 23 x H weights PER ELEMENT (tile layout [e][j][24] in global
-// memory): too large to stage for all D elements, so every warp streams the next element's block (H*24 + 23 floats)
-// into its own double buffer with cp.async while it works on the current element.
+// The same D-step sequential direction for a SPLINE masked autoregressive layer (MaskedAutoregressiveRQNSF /
+// MaskedAutoregressiveLRS sampling, InverseAutoregressiveRQNSF / InverseAutoregressiveLRS density).  The output layer is
+// P x H weights PER ELEMENT (tile layout [e][j][PP] in global memory; P = 23, PP = 24 for the rational-quadratic spline,
+// P = PP = 32 for the linear rational one): too large to stage for all D elements, so every warp streams the next element's
+// block (H*PP + P floats) into its own double buffer with cp.async while it works on the current element.
 // `xin`: where this layer reads its input row from (the kernel's input x for the first layer of an in-place program,
 // otherwise x0 itself); `live`: the thread owns a real row (threads past the end of the batch still take part in the
 // warp-wide weight staging but must not touch global memory).
@@ -310,7 +311,8 @@ template <int TK, int MODE, int HP>
 __device__ __forceinline__ void rows_sequential_rq(float* x0, const float* xin, bool live, int D, int rev, const DevOp& op,
                                                    const RowsWeights<HP>& W, const float* er, float* wst, int wst_stride,
                                                    float& ld) {
-    constexpr int P = 23, PP = 24;
+    constexpr int P = TInfo<TK>::P, PP = TInfo<TK>::PP;
+    constexpr bool LRS = TK == B2F_T_LRS_FWD || TK == B2F_T_LRS_INV;
     const int H = op.H, lane = threadIdx.x & 31;
     float pre[HP], act[HP];
     int fin[HP];
@@ -323,7 +325,7 @@ __device__ __forceinline__ void rows_sequential_rq(float* x0, const float* xin, 
     const bool quirk = !(op.flags & B2F_FLAG_SEQ_LOGDET_EXACT);
     // B2F_FLAG_SEQ_FOLDED: p[2] / p[3] hold the FOLDED output layer (24 columns per element, csrc/b2f_rqfast.cuh) and the
     // spline runs in the folded formulation of the tensor-core kernels: ~1/3 of the instructions of the stand-alone one
-    const bool folded = MODE != 0 && (op.flags & B2F_FLAG_SEQ_FOLDED);
+    const bool folded = !LRS && MODE != 0 && (op.flags & B2F_FLAG_SEQ_FOLDED);
     const float4* w1c = reinterpret_cast<const float4*>(W.w1);
     float* buf[2] = {wst, wst + wst_stride};
     auto stage = [&](int i, float* dst) {            // logical element i
@@ -381,7 +383,14 @@ __device__ __forceinline__ void rows_sequential_rq(float* x0, const float* xin, 
                 }
             }
         float out, l;
-        if (MODE != 0 && folded) {
+        if constexpr (LRS) {
+            transform_element<TK, MODE, PP>(v, acc, op.boundary, out, l);
+            if (quirk && i < D - 1) {
+                // the reference's last-iteration log-det (see below): the spline's log-det at the already inverted value
+                float out2;
+                transform_element<TK, MODE, PP>(out, acc, op.boundary, out2, l);
+            }
+        } else if (MODE != 0 && folded) {
             constexpr bool INV = TK == B2F_T_RQ_INV;
             if (quirk && i < D - 1) rqf::sequential_step<INV, true, true, (MODE >= 2)>(v, acc, op.boundary, out, l);
             else rqf::sequential_step<INV, true, false, (MODE >= 2)>(v, acc, op.boundary, out, l);
@@ -432,10 +441,12 @@ __device__ __forceinline__ void rows_layer(const float* wbuf, float* x0, int XS,
                                            const float* xin = nullptr, bool live = true) {
     if constexpr (RQ) {
         static_assert(R == 1, "spline layers: one row per thread");
-        if (op.tkind == B2F_T_RQ_FWD || op.tkind == B2F_T_RQ_INV) {       // sequential spline layer (host guarantees MADE_SEQ)
+        if (op.tkind == B2F_T_RQ_FWD || op.tkind == B2F_T_RQ_INV || op.tkind == B2F_T_LRS_INV) {
+            // sequential spline layer (host guarantees MADE_SEQ; linear rational splines: inverse direction only)
             const RowsWeights<HP> W = weights_view<HP>(wbuf, D);
             const float* in = xin ? xin : x0;
             if (op.tkind == B2F_T_RQ_INV) rows_sequential_rq<B2F_T_RQ_INV, MODE, HP>(x0, in, live, D, flip, op, W, er, wst, wst_stride, ld[0]);
+            else if (op.tkind == B2F_T_LRS_INV) rows_sequential_rq<B2F_T_LRS_INV, MODE, HP>(x0, in, live, D, flip, op, W, er, wst, wst_stride, ld[0]);
             else rows_sequential_rq<B2F_T_RQ_FWD, MODE, HP>(x0, in, live, D, flip, op, W, er, wst, wst_stride, ld[0]);
             return;
         }
@@ -517,6 +528,7 @@ __global__ void __launch_bounds__(NT) flow_rows_kernel(const __grid_constant__ R
             const int n_src = coupling ? D / 2 : D, n_tgt = coupling ? D - D / 2 : D;
             if (op.tkind == B2F_T_SHIFT_ADD || op.tkind == B2F_T_SHIFT_SUB) stage_weights<HP, 1, NT>(wbuf + A.woff[oi], op, n_src, n_tgt, seq, f);
             else if (op.tkind == B2F_T_RQ_FWD || op.tkind == B2F_T_RQ_INV) stage_weights<HP, 23, NT>(wbuf + A.woff[oi], op, n_src, n_tgt, seq, f);
+            else if (op.tkind == B2F_T_LRS_INV) stage_weights<HP, 32, NT>(wbuf + A.woff[oi], op, n_src, n_tgt, seq, f);
             else stage_weights<HP, 2, NT>(wbuf + A.woff[oi], op, n_src, n_tgt, seq, f);
         }
     }

@@ -1,5 +1,5 @@
 // Row-per-thread whole-flow kernel, instantiations for programs with sequential spline layers
-// (MaskedAutoregressiveRQNSF sampling, InverseAutoregressiveRQNSF density): device code in b2f_flow_rows.cuh
+// (MaskedAutoregressiveRQNSF / MaskedAutoregressiveLRS sampling, InverseAutoregressiveRQNSF / InverseAutoregressiveLRS density): device code in b2f_flow_rows.cuh
 // (rows_sequential_rq), eligibility and launch geometry in b2f_flow_rows.cu.  A separate translation unit only to
 // compile the spline variants in parallel with the affine ones.
 #include "b2f_flow_rows.cuh"
