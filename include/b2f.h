@@ -218,6 +218,14 @@ int64_t b2f_flow_backward_workspace(const b2f_op_t *ops, int32_t n_ops, int64_t 
  * else 0.  Only kind, tkind, n_hidden and n_bins of the ops are looked at, so callers can ask before any parameter exists
  * (torchflows_b200 decides at construction time whether a layer trains through the fused kernel or as a composite). */
 int32_t b2f_flow_backward_fits(const b2f_op_t *ops, int32_t n_ops, int32_t D);
+/* The tile shape b2f_flow_backward would launch for this program with these flags: returns 1 and writes out[0] = rows
+ * per tile TM, out[1] = threads per CTA NT and out[2] = the per-warp staging stride of a spline layer's output weights
+ * in floats (0: spline layers take the scalar GEMM path), or returns 0 if the kernel cannot take the program.  Host-only;
+ * honours B2F_FLOW_MODE_PRECISE and the environment overrides B2F_BWD_TM / B2F_BWD_NT / B2F_BWD_NO_MMA exactly as the
+ * launch does, so it tells whether a forced shape was admissible and fitted or fell back to the default one.  Looks at
+ * kind, tkind and n_hidden of the ops, and at the alignment of p[2] of spline layers (unaligned output weights disable
+ * the staging). */
+int32_t b2f_flow_backward_shape(const b2f_op_t *ops, int32_t n_ops, int32_t D, int32_t flags, int32_t out[3]);
 
 /* Elementwise transformer given materialised parameters h (TensorTransformer.forward / inverse,
  * transformers/base.py:24-42): x,out:(n_rows, n_event); h:(n_rows, n_event, P) with row stride

@@ -292,3 +292,86 @@ def test_bench_dump_outputs_fixed_row_sample(tmp_path):
     small = tmp_path / 'small'
     bench.dump_outputs(str(small), {'log_prob': lp[:100], 'sample': xs[:100]})
     assert np.array_equal(np.load(small / 'sample.npy'), xs[:100].numpy())
+
+
+def test_backward_tile_shape_query(monkeypatch):
+    """b2f_flow_backward_shape: the tile shape (rows per tile TM, threads NT, per-warp spline-weight staging) the fused
+    backward kernel launches, on the lowered programs of real presets.  Default-width presets climb a ladder of smaller
+    shapes as the shared-memory footprint grows with D, until the forward budget sends the layers to the composite path;
+    `precise` arithmetic turns the staging (tensor-core GEMM path) off; B2F_BWD_TM / B2F_BWD_NT force a shape when it is
+    admissible and fits, and are ignored otherwise."""
+    import torchflows_b200.architectures as arch
+    from torchflows_b200 import _native as N, _program as P
+    from torchflows_b200.bijections.finite.autoregressive.layers_base import _fits_fused_kernel
+    for var in ('B2F_BWD_TM', 'B2F_BWD_NT', 'B2F_BWD_NO_MMA'):
+        monkeypatch.delenv(var, raising=False)
+
+    def program(preset, D, **kwargs):
+        ops = getattr(arch, preset)(D, **kwargs).eval().fused_ops('forward')
+        assert ops is not None, (preset, D)
+        return P.op_dicts(ops)
+
+    def staging(ops):        # per-warp stride of one element's output weights + bias, H = widest spline layer <= 31
+        h = max([o['n_hidden'] for o in ops if o['kind'] in (N.OP_COUPLING, N.OP_MADE) and o['tkind'] == N.T_RQ_FWD
+                 and o['n_hidden'] <= 31], default=0)
+        return 24 * (h + 1) if h else 0
+
+    ladder = [('CouplingRQNSF', 64, 32, 384, True), ('CouplingRQNSF', 320, 32, 384, True),
+              ('CouplingRQNSF', 352, 32, 256, True), ('CouplingRQNSF', 448, 32, 256, True),
+              ('CouplingRQNSF', 480, 32, 128, True), ('CouplingRQNSF', 592, 32, 128, True),
+              ('CouplingRQNSF', 608, 32, 128, False),
+              ('RealNVP', 288, 64, 256, False), ('RealNVP', 304, 32, 256, False), ('RealNVP', 608, 32, 128, False),
+              ('MAF', 304, 64, 256, False), ('MAF', 320, 32, 256, False), ('MAF', 640, 32, 128, False),
+              ('MaskedAutoregressiveRQNSF', 480, 32, 384, True), ('MaskedAutoregressiveRQNSF', 496, 32, 256, True),
+              ('MaskedAutoregressiveRQNSF', 576, 32, 128, True),
+              ('CouplingLRS', 16, 64, 256, False), ('CouplingLRS', 272, 32, 256, False),
+              ('CouplingLRS', 560, 32, 128, False),
+              ('IAF', 320, 32, 256, False), ('InverseAutoregressiveRQNSF', 128, 64, 256, False)]
+    for preset, D, TM, NT, staged in ladder:
+        ops = program(preset, D)
+        want = (TM, NT, staging(ops) if staged else 0)
+        assert (not staged) or want[2] > 0, (preset, D)
+        assert N.flow_backward_shape(ops, D) == want, (preset, D, N.flow_backward_shape(ops, D), want)
+    # 608 still trains fused (on the scalar spline path); at 640 the forward budget sends the layers to the composite
+    assert _fits_fused_kernel(608, 19, N.OP_COUPLING, N.T_RQ_FWD, 8)
+    assert not _fits_fused_kernel(640, 19, N.OP_COUPLING, N.T_RQ_FWD, 8)
+    assert arch.CouplingRQNSF(640).eval().fused_ops('forward') is None
+
+    q256 = program('CouplingRQNSF', 256)
+    assert N.flow_backward_shape(q256, 256) == (32, 384, 24 * 18)
+    assert N.flow_backward_shape(q256, 256, N.FLOW_MODE_PRECISE) == (64, 256, 0)
+    wide_h = program('CouplingRQNSF', 64, conditioner_kwargs={'n_hidden': 32})
+    assert N.flow_backward_shape(wide_h, 64) == (64, 256, 0)
+    monkeypatch.setenv('B2F_BWD_NO_MMA', '1')
+    assert N.flow_backward_shape(q256, 256) == (64, 256, 0)
+    monkeypatch.delenv('B2F_BWD_NO_MMA')
+
+    spline, affine = program('CouplingRQNSF', 64), program('MAF', 64)
+    defaults = {id(spline): (32, 384, staging(spline)), id(affine): (64, 256, 0)}
+    for ops in (spline, affine):
+        assert N.flow_backward_shape(ops, 64) == defaults[id(ops)]
+        for TM, NT in ((32, 32), (32, 160), (64, 64), (64, 192), (64, 384)):
+            monkeypatch.setenv('B2F_BWD_TM', str(TM))
+            monkeypatch.setenv('B2F_BWD_NT', str(NT))
+            assert N.flow_backward_shape(ops, 64) == (TM, NT, defaults[id(ops)][2]), (TM, NT)
+        for TM, NT in ((64, 32), (48, 256), (32, 416), (64, 416)):        # NT < TM, TM not a power of two, NT > 384
+            monkeypatch.setenv('B2F_BWD_TM', str(TM))
+            monkeypatch.setenv('B2F_BWD_NT', str(NT))
+            assert N.flow_backward_shape(ops, 64) == defaults[id(ops)], (TM, NT)
+    # admissible but too large for the program: 64 x 384 with staging does not fit beside CouplingRQNSF(256)'s tiles
+    monkeypatch.setenv('B2F_BWD_TM', '64')
+    monkeypatch.setenv('B2F_BWD_NT', '384')
+    assert N.flow_backward_shape(q256, 256) == (32, 384, 24 * 18)
+    monkeypatch.delenv('B2F_BWD_TM')
+    monkeypatch.delenv('B2F_BWD_NT')
+
+    # b2f_flow_backward_fits answers for one layer what the query answers at flags = 0
+    for kind, tkind in ((N.OP_COUPLING, N.T_RQ_FWD), (N.OP_COUPLING, N.T_AFFINE_FWD), (N.OP_MADE, N.T_RQ_FWD),
+                        (N.OP_MADE_SEQ, N.T_AFFINE_INV), (N.OP_COUPLING, N.T_LRS_FWD)):
+        for H in (4, 19, 31, 32, 64, 1024):
+            for D in (16, 256, 608, 640, 768, 1024, 2048, 4096):
+                n_bins = 8 if tkind in (N.T_RQ_FWD, N.T_LRS_FWD) else 0
+                op = [dict(kind=kind, tkind=tkind, n_hidden=H, n_bins=n_bins)]
+                fits = N.flow_backward_fits(kind, tkind, H, n_bins, D)
+                assert fits == (N.flow_backward_shape(op, D) is not None), (kind, tkind, H, D)
+    assert N.flow_backward_shape([dict(kind=N.OP_COUPLING, tkind=N.T_RQ_FWD, n_hidden=1024, n_bins=8)], 4096) is None

@@ -83,6 +83,8 @@ def lib():
         L.b2f_flow_backward_workspace.restype = i64
         L.b2f_flow_backward_fits.argtypes = [ctypes.POINTER(Op), i32, i32]
         L.b2f_flow_backward_fits.restype = i32
+        L.b2f_flow_backward_shape.argtypes = [ctypes.POINTER(Op), i32, i32, i32, ctypes.POINTER(i32 * 3)]
+        L.b2f_flow_backward_shape.restype = i32
         L.b2f_transformer_apply.argtypes = [i32, vp, vp, vp, vp, vp, i64, i32, i64, i32, f32, i32, vp]
         L.b2f_transformer_backward.argtypes = [i32, vp, vp, vp, vp, vp, vp, i64, i32, i64, i32, f32, i32, vp]
         L.b2f_column_stats.argtypes = [vp, vp, vp, i64, i32, vp]
@@ -203,6 +205,17 @@ def flow_backward_fits(kind: int, tkind: int, n_hidden: int, n_bins: int, D: int
     arr = (Op * 1)()
     arr[0].kind, arr[0].tkind, arr[0].n_hidden, arr[0].n_bins = kind, tkind, n_hidden, n_bins
     return bool(lib().b2f_flow_backward_fits(arr, 1, D))
+
+
+def flow_backward_shape(ops: Sequence[dict], D: int, flags=0):
+    """(TM, NT, wst_stride) that flow_backward would launch for this program, or None if the backward kernel cannot take
+    it.  wst_stride > 0: spline layers take the tensor-core GEMM path.  Host-only; honours the B2F_BWD_TM / B2F_BWD_NT /
+    B2F_BWD_NO_MMA overrides and FLOW_MODE_PRECISE in `flags` as the launch does."""
+    arr = make_ops(ops)
+    out = (ctypes.c_int32 * 3)()
+    if not lib().b2f_flow_backward_shape(arr, len(ops), D, flags, ctypes.byref(out)):
+        return None
+    return tuple(out)
 
 
 def last_flow_kernel() -> int:

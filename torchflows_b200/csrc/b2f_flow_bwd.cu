@@ -860,6 +860,15 @@ extern "C" int32_t b2f_flow_backward_fits(const b2f_op_t* ops, int32_t n_ops, in
     return bwd_tile_shape(ops, n_ops, D, 0, shape) ? 1 : 0;
 }
 
+extern "C" int32_t b2f_flow_backward_shape(const b2f_op_t* ops, int32_t n_ops, int32_t D, int32_t flags, int32_t out[3]) {
+    if (!ops || n_ops < 0 || n_ops > B2F_MAX_OPS || D <= 0 || !out) return 0;
+    if (getenv("B2F_BWD_NO_MMA")) flags |= B2F_FLOW_MODE_PRECISE;     // as b2f_flow_backward does
+    BwdShape shape;
+    if (!bwd_tile_shape(ops, n_ops, D, flags, shape)) return 0;
+    out[0] = shape.TM; out[1] = shape.NT; out[2] = shape.wst_stride;
+    return 1;
+}
+
 extern "C" int b2f_flow_backward(const b2f_op_t* ops, int32_t n_ops, const float* x, const float* gy,
                                  const float* glog_det, const float* glog_prob, const float* base_loc,
                                  const float* base_log_scale, float* gx, void* workspace, int64_t B, int32_t D,
