@@ -100,7 +100,8 @@ enum b2f_op_kind {
                                                 (maps the written value to the standardised base-density argument; 0 unless this
                                                 layer is the last writer of the column), 0, 0
                                          src    [Dh][2]: a, b of the pending elementwise layers on the source half
-                                         misc   [4]: sup |log2e*u_x|, sup |log2e*u_y/1000| over all inputs (from the weights), 0, 0
+                                         misc   [4]: sup |log2e*u_x|, sup |log2e*u_y/1000|, sup |u_d/1000| over all inputs (from the weights;
+                                                      the last includes the padded edge logit c/1000, 0 = no bound), 0
                                        p[5] (first coupling op) = program blob: int32 {magic, final pass on half 0, on half 1, layers},
                                          {sum of elementwise log-dets, base-density constant, 0, 0}, [D][2] final affine per physical
                                          column, [D][2] (exp(-log_scale), -loc*exp(-log_scale)) of the base density per column */

@@ -93,6 +93,17 @@ def fold_output_layer(W2: torch.Tensor, b2: torch.Tensor, Dh: int):
     return Wf.float(), bf.float()
 
 
+def derivative_logit_bound(W2: torch.Tensor, b2: torch.Tensor, Dh: int) -> torch.Tensor:
+    """sup |a - c| over all inputs and knots of the padded derivative logits a = c + [c, u_d, c]/1000 (|tanh| <= 1, so
+    |u_d| <= sum_h |w| + |b| on the unfolded derivative rows): admits csrc/b2f_rqfast.cuh delta_poly when below
+    kDeltaPolyBound.  Never 0 (the edge logits contribute c/1000), which the kernel reads as "no bound"."""
+    H = W2.shape[1]
+    w = W2.reshape(Dh, 23, H)[:, 16:23].double()
+    b = b2.reshape(Dh, 23)[:, 16:23].double()
+    interior = (w.abs().sum(dim=2) + b.abs()).max() / 1000.0
+    return torch.clamp(interior, min=abs(RQ_EDGE_U) / 1000.0).float()
+
+
 def _elementwise_affine(op, flip: bool):
     """(a, b, sum log|a|) of one ElementwiseAffine / ActNorm op as z = a*x + b per PHYSICAL column
     (affine.py:33-59; layers_base.py:300-318)."""
@@ -155,12 +166,13 @@ def build_plan(ops: Sequence, D: int, base_loc: Optional[torch.Tensor], base_log
                 t = 1 - s
                 W1, b1, W2, b2 = (x.detach().float() for x in op.leafs)
                 H = W1.shape[0]
+                bound_d = derivative_logit_bound(W2, b2, Dh)
                 layer = dict(src_half=s, tgt_half=t, src_pass=pending[s], H=H, K2=(H + 2 + 7) // 8 * 8,
                              boundary=float(op.boundary), inverse=op.tkind == N.T_RQ_INV,
                              src_a=A[half[s]].clone(), src_b=B[half[s]].clone(),
                              pre_a=A[half[t]].clone(), pre_b=B[half[t]].clone(),
                              post_a=torch.ones(Dh, **f32), post_b=torch.zeros(Dh, **f32),
-                             W1=(W1.flip(1) if flip else W1), b1=b1)
+                             W1=(W1.flip(1) if flip else W1), b1=b1, bound_d=bound_d)
                 Wf, bf = fold_output_layer(W2, b2, Dh)
                 if flip:                      # physical order of the target columns is the reverse of the logical one
                     Wf, bf = Wf.flip(0), bf.flip(0)
@@ -211,7 +223,7 @@ def build_plan(ops: Sequence, D: int, base_loc: Optional[torch.Tensor], base_log
             sp = torch.stack([layer['src_a'], layer['src_b']], dim=1).reshape(-1)
             # |tanh| <= 1, so |column| <= sum_h |w| + |b|: proves the ranges the fast spline variant relies on
             absum = layer['Wf'].abs().sum(dim=2) + layer['bf'].abs()
-            misc = torch.stack([absum[:, 0:8].max(), absum[:, 8:16].max(), torch.zeros((), **f32), torch.zeros((), **f32)])
+            misc = torch.stack([absum[:, 0:8].max(), absum[:, 8:16].max(), layer['bound_d'], torch.zeros((), **f32)])
             layer['bound_L'], layer['bound_Dl'] = misc[0], misc[1]
             layer['M'] = M
             blob = torch.cat([hdr, canonical(W1p), b1p, w2c, tp, sp, misc]).contiguous()

@@ -67,6 +67,7 @@ struct QArgs {
     const float* prog;      // program blob: [4 ints][4 consts][D x (fin_a, fin_b)][D x (in_a, in_b)]
     // Flow.sample with in-kernel noise (b2f_flow_sample): the input tile is drawn from the Philox stream instead of loaded
     int philox;
+    int no_dpoly;           // B2F_TCQ_NO_DPOLY: SFU softplus for the knot derivatives even where delta_poly is admitted
     unsigned long long seed, offset;
     const float* base_loc;          // nullable: standard normal
     const float* base_log_scale;
@@ -150,10 +151,12 @@ __device__ __forceinline__ void q_affine_pass(uint32_t half_addr, uint32_t row_o
 }
 
 // One coupling layer's transformer phase for one epilogue thread (row m, group g): its chunks c = g, g + 4, ...
-template <bool INV, bool SAFE>
+// DPOLY: knot derivatives from rqf::delta_poly.  LD = false (inverse only): the transformed values alone, ld2 and sq untouched.
+template <bool INV, bool SAFE, bool DPOLY, bool LD>
 __device__ __forceinline__ void q_chunk_loop(const QSmem& s, const float* __restrict__ tp, float boundary, uint32_t tbase,
                                              uint32_t lane_addr, uint32_t tgt_addr, int Dh, int n_chunks, uint32_t cc_base, int m,
                                              int g, int lane, float& ld2, float& sq) {
+    static_assert(INV || LD, "the forward direction always feeds a log-density");
     const uint32_t xrow = tgt_addr + (m >> 3) * (Dh * 32) + (m & 7) * 16;       // canon_off(m, 0, Dh)
     for (int c = g; c < n_chunks; c += 4) {
         const uint32_t ccl = cc_base + c, slot = ccl & (kQSlots - 1);
@@ -181,14 +184,15 @@ __device__ __forceinline__ void q_chunk_loop(const QSmem& s, const float* __rest
         float oa, ob, la, lb;
         const float va = fmaf(xv.x, pa.x, pa.y), vb = fmaf(xv.y, pb.x, pb.y);
         if (INV) {
-            rqf::inverse<SAFE, B2F_TCQ_NY>(va, ga, boundary, oa, la);
-            rqf::inverse<SAFE, B2F_TCQ_NY>(vb, gb, boundary, ob, lb);
+            rqf::inverse<SAFE, B2F_TCQ_NY, DPOLY, LD>(va, ga, boundary, oa, la);
+            rqf::inverse<SAFE, B2F_TCQ_NY, DPOLY, LD>(vb, gb, boundary, ob, lb);
         } else {
-            rqf::forward<SAFE, B2F_TCQ_NY>(va, ga, boundary, oa, la);
-            rqf::forward<SAFE, B2F_TCQ_NY>(vb, gb, boundary, ob, lb);
+            rqf::forward<SAFE, B2F_TCQ_NY, DPOLY>(va, ga, boundary, oa, la);
+            rqf::forward<SAFE, B2F_TCQ_NY, DPOLY>(vb, gb, boundary, ob, lb);
         }
         const float sa = fmaf(oa, pa.z, pa.w), sb = fmaf(ob, pb.z, pb.w);
         q_sts64(px, make_float2(sa, sb));
+        if (!LD) continue;
         const float ta = fmaf(sa, fa.x, fa.y), tb = fmaf(sb, fb.x, fb.y);
         sq = fmaf(ta, ta, sq);
         sq = fmaf(tb, tb, sq);
@@ -200,6 +204,9 @@ __device__ __forceinline__ void q_chunk_loop(const QSmem& s, const float* __rest
 // alternates from tile to tile (`swap`), because the next tile is prefetched half by half into whatever the current tile
 // releases first: the source half of the LAST layer is dead once that layer's GEMM1 has read it (EARLY_FREE) and receives
 // the next tile's FIRST-layer source half; the other half follows when the tile is done (TILE_DONE).
+// LD = false: Flow.sample without log_prob -- neither log-det nor log-density is written, so the inverse layers compute the
+// transformed values only and the per-tile reduction is skipped.  Launched only on programs whose layers are all inverse.
+template <bool LD>
 __global__ void __launch_bounds__(kQThreads, 1)
 flow_tcq_kernel(const __grid_constant__ QArgs A, const __grid_constant__ CUtensorMap map_x,
                 const __grid_constant__ CUtensorMap map_y) {
@@ -511,21 +518,29 @@ flow_tcq_kernel(const __grid_constant__ QArgs A, const __grid_constant__ CUtenso
                     if (lane == 0) umma::mbar_arrive(&s.bars[QB_EARLY_FREE]);
                 }
                 if (!have_b) { umma::mbar_wait(&s.bars[QB_XB_FULL], tc & 1); have_b = true; }
-                // transformer phase
+                // transformer phase.  misc[2] = 0 means no bound on the derivative logits (it is never 0 otherwise: it
+                // includes the padded edge logit)
                 const bool fast = __ldg(misc) < rqf::kNoMaxBound && __ldg(misc + 1) < rqf::kPolyBound;
-                if (L.inverse) {
-                    if (fast) q_chunk_loop<true, false>(s, tp, L.boundary, tbase, lane_addr, tgt_addr, Dh, n_chunks, cc, m, g, lane, ld2, sq);
-                    else q_chunk_loop<true, true>(s, tp, L.boundary, tbase, lane_addr, tgt_addr, Dh, n_chunks, cc, m, g, lane, ld2, sq);
+                const float bound_d = __ldg(misc + 2);
+                const bool dpoly = fast && !A.no_dpoly && bound_d > 0.0f && bound_d < rqf::kDeltaPolyBound;
+#define B2F_Q_CHUNKS(INV, SAFE, DPOLY, LDV) \
+    q_chunk_loop<INV, SAFE, DPOLY, LDV>(s, tp, L.boundary, tbase, lane_addr, tgt_addr, Dh, n_chunks, cc, m, g, lane, ld2, sq)
+                if (LD && !L.inverse) {
+                    if (dpoly) B2F_Q_CHUNKS(false, false, true, true);
+                    else if (fast) B2F_Q_CHUNKS(false, false, false, true);
+                    else B2F_Q_CHUNKS(false, true, false, true);
                 } else {
-                    if (fast) q_chunk_loop<false, false>(s, tp, L.boundary, tbase, lane_addr, tgt_addr, Dh, n_chunks, cc, m, g, lane, ld2, sq);
-                    else q_chunk_loop<false, true>(s, tp, L.boundary, tbase, lane_addr, tgt_addr, Dh, n_chunks, cc, m, g, lane, ld2, sq);
+                    if (dpoly) B2F_Q_CHUNKS(true, false, true, LD);
+                    else if (fast) B2F_Q_CHUNKS(true, false, false, LD);
+                    else B2F_Q_CHUNKS(true, true, false, LD);
                 }
+#undef B2F_Q_CHUNKS
                 cc += n_chunks;
             }
             // ---- outputs of this tile ----
-            s.red[g * 128 + m] = make_float2(ld2, sq);
-            q_epi_sync();
-            if (tid < 128) {
+            if (LD) s.red[g * 128 + m] = make_float2(ld2, sq);
+            q_epi_sync();                         // also orders the last layer's writes before the passes over the tile
+            if (LD && tid < 128) {
                 const float2 r0 = s.red[tid], r1 = s.red[128 + tid], r2 = s.red[256 + tid], r3 = s.red[384 + tid];
                 const float ld = fmaf((r0.x + r1.x) + (r2.x + r3.x), rqf::kLn2, const_ld);
                 float sqs = (r0.y + r1.y) + (r2.y + r3.y);
@@ -647,13 +662,19 @@ int try_launch_flow_tcq(const b2f_op_t* ops, int32_t n_ops, const float* x, floa
     }
     if (A.use_tma && !noise && !make_tile_map(&map_x, x, B, D)) A.use_tma = 0;
     if (A.use_tma && y && !make_tile_map(&map_y, y, B, D)) A.use_tma = 0;
+    A.no_dpoly = getenv("B2F_TCQ_NO_DPOLY") ? 1 : 0;
+    // the output-only kernel when nothing reads the log-det (Flow.sample without log_prob) and every layer is inverse
+    bool ld = log_det || log_prob || getenv("B2F_TCQ_ALWAYS_LD");
+    for (int i = 0; i < A.n_layers; ++i) ld = ld || !A.layers[i].inverse;
     int dev = 0, n_sm = 148;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev);
     const int grid = std::min(A.n_tiles, n_sm);
-    cudaError_t ce = (cudaError_t)raise_smem_limit((const void*)flow_tcq_kernel, smem);
+    const void* kfn = ld ? (const void*)flow_tcq_kernel<true> : (const void*)flow_tcq_kernel<false>;
+    cudaError_t ce = (cudaError_t)raise_smem_limit(kfn, smem);
     if (ce != cudaSuccess) return fail(B2F_ERR_CUDA, "cudaFuncSetAttribute(tcq): %s", cudaGetErrorString(ce));
-    flow_tcq_kernel<<<grid, kQThreads, smem, (cudaStream_t)stream>>>(A, map_x, map_y);
+    if (ld) flow_tcq_kernel<true><<<grid, kQThreads, smem, (cudaStream_t)stream>>>(A, map_x, map_y);
+    else flow_tcq_kernel<false><<<grid, kQThreads, smem, (cudaStream_t)stream>>>(A, map_x, map_y);
     const int rc = check_launch("b2f_flow_apply (spline tensor-core kernel)");
     return rc == B2F_OK ? 1 : rc;
 }

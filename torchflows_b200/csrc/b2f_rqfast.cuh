@@ -17,7 +17,10 @@
 //  * heights softmax: exp(L + Dl) = exp(L) * 2^Dl with a cubic for 2^Dl when the host proves |Dl| < 1/32 from the
 //    weights (|tanh| <= 1), else the SFU;  no max-subtraction when the host proves |L| < 40 (same bound);
 //  * one reciprocal for both softmax normalisations, one for the rational function (everything multiplied through by
-//    w^3), one lg2 for the log-determinant;  the log-det is returned in log2 units and scaled once per row.
+//    w^3), one lg2 for the log-determinant;  the log-det is returned in log2 units and scaled once per row;
+//  * knot derivatives: a cubic for softplus when the host proves |a - c| < 1/32 from the weights (DPOLY), else the SFU;
+//  * the inverse map can skip its log-determinant altogether (LD = false: Flow.sample without log_prob); the output chain
+//    never reads the log-det arithmetic, so `out` is bit-identical either way.
 //
 // Tolerance-checked (1e-4 abs/rel on log_prob), not bit-checked: the bit-exact bin index contract belongs to the
 // stand-alone transformer kernel (b2f_math.cuh), whose parameters are fp32-faithful; here they come out of a TF32 GEMM.
@@ -33,6 +36,9 @@ constexpr float kSizeScale = 0.992f;          // 1 - 1e-3 * 8   (rational_quadra
 constexpr float kPolyBound = 1.0f / 32.0f;    // |Dl| below which the cubic 2^Dl is exact to 1e-8
 constexpr float kNoMaxBound = 40.0f;          // |L| below which ex2 needs no max subtraction
 constexpr float kEdgeLogit = kRqEdgeU + kRqEdgeU / 1000.0f;   // logit of the two padded edge derivatives: c + c/1000
+// |a - c| (derivative logit a, c = kRqEdgeU) below which delta_poly is within 1 ulp of the exact delta: the cubic's
+// truncation error is < 4e-9 there, the rest is the rounding of the last FMA (tests/test_tcq_specialise_host.py)
+constexpr float kDeltaPolyBound = 1.0f / 32.0f;
 
 B2F_HD float f_ex2(float x) {
 #if defined(__CUDA_ARCH__)
@@ -69,9 +75,24 @@ B2F_HD float delta(float a) {
     return fmaf(f_lg2(1.0f + e), kLn2, kRqMinDelta);
 }
 
+// delta at the two knot logits kRqEdgeU + u.x, kRqEdgeU + u.y for |u| < kDeltaPolyBound: Taylor cubic of 1e-5 + softplus
+// around c = kRqEdgeU, coefficients in fp64 at the fp32 value of c.  softplus(c) = 1 - 1e-5 (rational_quadratic.py:38), so
+// the constant term is 1 (1 + 1.5e-8 in fp64).  The first step is two scalar FMAs: they take both coefficients as
+// immediates, where FFMA2 would hold its multiplier in a register across the chunk loop (+2 registers in the sampling kernel).
+B2F_HD f2 delta_poly(f2 u) {
+    f2 p = mk2(fmaf(u.x, -0.01024104604576881f, 0.1162725642742006f), fmaf(u.y, -0.01024104604576881f, 0.1162725642742006f));
+    p = pk_fma(p, u, mk2(0.6321168855657702f, 0.6321168855657702f));
+    return pk_fma(p, u, mk2(1.0f, 1.0f));
+}
+
 struct Sel {            // the selected bin: knots measured from -b (cumulative bin sizes in [0, 2b]), derivative logits
-    float xl, xu, yl, yu, dl0, dl1;
+    float xl, xu, yl, yu, dl0, dl1;     // DPOLY: dl0, dl1 are the logits minus kRqEdgeU
 };
+
+template <bool DPOLY>
+B2F_HD f2 knot_deltas(const Sel& s) {
+    return DPOLY ? delta_poly(mk2(s.dl0, s.dl1)) : mk2(delta(s.dl0), delta(s.dl1));
+}
 
 // One search step with the predicate as a number, m = (c < t) ? 1 : 0:  lo += m a, up += m b (packed pairs),
 // dl0 += m d0, dl1 += m d1.  fma(1, x, acc) rounds exactly like acc + x, so this IS the predicated sum; as FFMA2 / FFMA
@@ -89,8 +110,9 @@ B2F_HD float select_step(float c, float t, f2& lo, f2& up, float& dl0, float& dl
 // Softmaxes, search and selection.  t = v + b.  INV: search on the y knots (rational_quadratic.py:147).
 // SAFE: max-subtracted exponentials and SFU for the heights (no host-side bound on the logits).
 // NY (even): how many of the 8 heights exponentials go to the SFU in the fast variant (pipe balancing; any value is exact).
+// DPOLY: derivative logits accumulated relative to kRqEdgeU (the offsets delta_poly takes).
 // Widths and heights travel as packed pairs (.x widths, .y heights): FADD2 / FFMA2 issue once for both.
-template <bool INV, bool SAFE, int NY>
+template <bool INV, bool SAFE, int NY, bool DPOLY = false>
 B2F_HD void select(const float (&g)[24], float t, float two_b, Sel& s) {
     static_assert(NY % 2 == 0, "the cubic 2^d is evaluated on pairs of logits");
     f2 e[8];
@@ -126,7 +148,8 @@ B2F_HD void select(const float (&g)[24], float t, float two_b, Sel& s) {
 #pragma unroll
     for (int j = 0; j < 8; ++j) sz[j] = pk_fma(e[j], rr, mk2(minb, minb));
     f2 lo = mk2(0.0f, 0.0f), up = sz[0];
-    s.dl0 = kEdgeLogit; s.dl1 = kEdgeLogit + g[16];
+    const float edge = DPOLY ? kRqEdgeU / 1000.0f : kEdgeLogit;
+    s.dl0 = edge; s.dl1 = edge + g[16];
     float c = 0.0f, m7 = 0.0f;
 #pragma unroll
     for (int j = 1; j < 8; ++j) {
@@ -139,17 +162,18 @@ B2F_HD void select(const float (&g)[24], float t, float two_b, Sel& s) {
 }
 
 // Forward map (rational_quadratic.py:88-109, log-det :56-63).  out = spline(v), ld2 = log2 |d out / d v|.
-template <bool SAFE, int NY>
+template <bool SAFE, int NY, bool DPOLY = false>
 B2F_HD void forward(float v, const float (&g)[24], float b, float& out, float& ld2) {
     const float two_b = b + b;
     const bool inb = fabsf(v) < b;                        // strict, spline/base.py:29-33; NaN -> identity tail
     const float t = v + b;
     Sel s;
-    select<false, SAFE, NY>(g, t, two_b, s);
+    select<false, SAFE, NY, DPOLY>(g, t, two_b, s);
     const float w = s.xu - s.xl, hgt = s.yu - s.yl;
     const float yk = s.yl - b;
     const float a = fminf(fmaxf(t - s.xl, 0.0f), w);      // v - x_k = xi * w, xi clipped to [0, 1]  (:99)
-    const float d0 = delta(s.dl0), d1 = delta(s.dl1);
+    const f2 dd = knot_deltas<DPOLY>(s);
+    const float d0 = dd.x, d1 = dd.y;
     // out = yk + hgt (s xi^2 + d0 q) / (s + t1 q), everything multiplied through by w^3:
     const float wa = w - a, aw = a * wa, h2 = hgt + hgt;
     const float T = fmaf(w, d0 + d1, -h2);                // w * t1
@@ -165,17 +189,19 @@ B2F_HD void forward(float v, const float (&g)[24], float b, float& out, float& l
 }
 
 // Inverse map (rational_quadratic.py:153-181).  out = spline^{-1}(v), ld2 = -log2 |d spline / d x| at out.
-template <bool SAFE, int NY>
+// LD = false: out only, ld2 is not written.
+template <bool SAFE, int NY, bool DPOLY = false, bool LD = true>
 B2F_HD void inverse(float v, const float (&g)[24], float b, float& out, float& ld2) {
     const float two_b = b + b;
     const bool inb = fabsf(v) < b;
     const float t = v + b;
     Sel s;
-    select<true, SAFE, NY>(g, t, two_b, s);
+    select<true, SAFE, NY, DPOLY>(g, t, two_b, s);
     const float w = s.xu - s.xl, hgt = s.yu - s.yl;
     const float xk = s.xl - b;
     const float t0 = fminf(fmaxf(t - s.yl, 0.0f), hgt);   // v - y_k
-    const float d0 = delta(s.dl0), d1 = delta(s.dl1);
+    const f2 dd = knot_deltas<DPOLY>(s);
+    const float d0 = dd.x, d1 = dd.y;
     const float h2 = hgt + hgt, hw = hgt * w;
     const float T = fmaf(w, d0 + d1, -h2);                // w * t1
     // quadratic of :170-178 multiplied by w:  A = hgt^2 - B,  B = hgt d0 w - t0 T,  C = -hgt t0
@@ -184,13 +210,14 @@ B2F_HD void inverse(float v, const float (&g)[24], float b, float& out, float& l
     const float disc = fmaf(B2, B2, (4.0f * (A2 * hgt)) * t0);
     const float sq = f_sqrt(fmaxf(disc, 0.0f));
     const float xi = fminf(fmaxf((h2 * t0) * f_rcp(B2 + sq), 0.0f), 1.0f);
+    const float o = fmaf(xi, w, xk);                      // one explicit FMA: the same rounding with and without LD
+    out = inb ? o : v;
+    if (!LD) return;
     const float a = xi * w;
-    const float o = xk + a;
     const float wa = w - a, aw = a * wa;
     const float den = fmaf(T, aw, hw * w);
     const float M3 = fmaf(w, fmaf(d0 * wa, wa, (d1 * a) * a), h2 * aw);
     const float fw = (hgt * hgt) * (M3 * w);              // forward derivative = fw / den^2
-    out = inb ? o : v;
     ld2 = f_lg2(inb ? den * den : 1.0f) - f_lg2(inb ? fw : 1.0f);
 }
 
